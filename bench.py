@@ -23,6 +23,9 @@ s_per_explained_query: wall time of Explainer(...).run(q, 1) through the drop-in
 cpu_baseline / --impl reference: the unmodified reference's kernel_output (perturbator + Model.infer; PyG layers from the
           CPU stand-in because torch_geometric is absent) on the host cores, bounded sample; the oracle port when the staged
           reference is missing.  The parity check of the run: exit code 3 when GPU and CPU disagree beyond the bar.
+--dump-outputs DIR: the predictions of the last timed step as DIR/predictions.npy, coalition rows x queries (inputs are
+          seeded: equal arguments give equal inputs, so two builds can be compared output for output).  --impl reference
+          evaluates the first query only, so its file has one column.
 """
 import argparse
 import json
@@ -380,10 +383,12 @@ def run_reference(args, rank):
     times, kind = [], "port"
     for i in range(args.steps + args.warmup):
         t0 = time.perf_counter()
-        _, kind = host_eval(wl, om, mask[i * b:(i + 1) * b], ref)
+        y, kind = host_eval(wl, om, mask[i * b:(i + 1) * b], ref)
         dt = time.perf_counter() - t0
         if i >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, np.reshape(y, (b, -1)))
     t = float(np.sum(times))
     value = b * len(times) / t
     line = {
@@ -573,6 +578,23 @@ def emit(line):
     _REAL_STDOUT.flush()
 
 
+DUMP_BYTES = 64 << 20  # --dump-outputs writes at most this much
+
+
+def dump_outputs(out_dir, y):
+    """Writes the predictions of the last timed step (coalition rows x queries) as ``predictions.npy`` (float32) so that
+    two builds can be compared output for output; the inputs are seeded, so equal arguments give equal inputs.  Beyond
+    DUMP_BYTES a fixed, seeded sample of the rows is written, and their indices as ``prediction_rows.npy`` (float64)."""
+    y = np.ascontiguousarray(y, dtype=np.float32)
+    os.makedirs(out_dir, exist_ok=True)
+    row_bytes = y[0].nbytes + 8
+    if y.nbytes > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(y.shape[0], (DUMP_BYTES - 4096) // row_bytes, replace=False))
+        y = y[rows]
+        np.save(os.path.join(out_dir, "prediction_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "predictions.npy"), y)
+
+
 PARITY_BAR = {"fp32": 1e-4, "bf16": 2e-2, "bf16_act": 2e-2}  # BASELINE.json north_star tolerances on the predictions
 PARITY_ATOL = 1e-6  # absolute floor for predictions that are themselves ~0 (cancelling head sums): the tests' Y_ATOL
 
@@ -593,7 +615,11 @@ def main():
     ap.add_argument("--precision", default="fp32", choices=["fp32", "bf16", "bf16_act"],
                     help="fp32: TF32x3 tensor-core transforms (1e-4 parity bar); bf16: bf16 transforms (2e-2 bar); "
                          "bf16_act: bf16 transforms and bf16 activation storage (2e-2 bar)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the predictions of the last timed step (coalitions x queries; "
+                                                         "--impl reference: the first query only) to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         os.environ["CUDA_VISIBLE_DEVICES"] = ""  # the reference takes its cupy branch when CUDA is visible (data.py:431)
     _claim_stdout()
@@ -668,6 +694,9 @@ def main():
             y = forward(act, record=True)
         ev1.record()
         barrier()
+    if args.dump_outputs and rank == 0:  # rank 0 holds every rank's rows after the all-gather, each padded to s_max
+        y_last = y.cpu().numpy().reshape(world, -1, nq) if world > 1 else y.cpu().numpy()[None]
+        y_last = np.concatenate([y_last[r, :rows[r]] for r in range(world)])
     ms_rank = float(ev0.elapsed_time(ev1))
     compute_rank = float(sum(a.elapsed_time(b) for a, b in compute_events))
     ms_all = torch.tensor([ms_rank, compute_rank], device=dev)
@@ -700,6 +729,8 @@ def main():
 
     rc = 0
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, y_last)
         evals = s_total * args.steps * nq  # SURVEY.md 8d: coalition rows x queries
         value = evals / (ms_total / 1e3)
         visits = eng.edge_visits_per_coalition  # kept edges x conv layers

@@ -74,15 +74,17 @@ def test_rmat_generator_is_skewed_and_in_range():
     assert int(indeg.max()) > 20 * float(indeg.float().mean())  # hub rows
 
 
-def test_reference_arm_prints_one_contract_line():
+def test_reference_arm_prints_one_contract_line(tmp_path):
     """`bench.py --impl reference` (the unmodified reference's kernel_output where the reference tree or its staged copy
-    exists, else the oracle port) prints ONE JSON line with the contract keys; it must work without a GPU."""
+    exists, else the oracle port) prints ONE JSON line with the contract keys and writes the predictions of its last step
+    with --dump-outputs; it must work without a GPU."""
     import json
     import subprocess
 
     env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--workload", "tiny", "--steps", "1",
-                          "--warmup", "0", "--ref-coalitions", "2", "--no-query-leg"], capture_output=True, text=True, env=env, timeout=600)
+                          "--warmup", "0", "--ref-coalitions", "2", "--no-query-leg", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, env=env, timeout=600)
     assert out.returncode == 0, out.stderr[-2000:]
     lines = [l for l in out.stdout.splitlines() if l.strip()]
     assert len(lines) == 1
@@ -91,6 +93,8 @@ def test_reference_arm_prints_one_contract_line():
     assert d["value"] > 0 and d["higher_is_better"] is True and d["config"]["workload"] == "tiny"
     assert d["cpu_baseline"]["kind"] in ("reference", "port") and d["cpu_baseline"]["value"] == d["value"]
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
+    y = np.load(tmp_path / "predictions.npy")
+    assert y.shape == (2, 1) and y.dtype == np.float32 and np.isfinite(y).all()
 
 
 def test_reference_and_port_agree_on_the_bench_workload():

@@ -681,3 +681,26 @@ def test_parity_at_bench_scale(name, lib, knobs):
     tile = MaskedForward(eng.graph, lower(arch), [q], prune=False, zero_edge_rule=wl.kind == "hetero_sage")
     yt = tile(act, 8)[:, 0].cpu().numpy()
     assert rel(yt) <= 1e-4, ("tile path", rel(yt))
+
+
+def test_bench_dump_outputs_are_the_timed_predictions(lib, tmp_path):
+    """``bench.py --dump-outputs`` writes the predictions of its timed path: one row per coalition of the job (40 rows:
+    the second 32-row word is partial), equal to the oracle on the same seeded coalitions, regenerated here with
+    bench.make_packed_masks and bench's seed of rank 0."""
+    import subprocess
+
+    sys.path.insert(0, ROOT)
+    import bench
+
+    rows = 40
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "tiny", "--coalitions", str(rows),
+                          "--steps", "2", "--warmup", "1", "--no-query-leg", "--no-cpu-baseline", "--dump-outputs",
+                          str(tmp_path)], capture_output=True, text=True, timeout=900)
+    assert out.returncode == 0, out.stderr[-2000:]
+    y = np.load(tmp_path / "predictions.npy")
+    wl = bench.Workload("tiny")
+    assert y.shape == (rows, len(wl.queries)) and y.dtype == np.float32
+    _, sample = bench.make_packed_masks(lib, rows, wl.n, wl.c, wl.com_of, 1000, torch.device("cuda", 0), wl.com_of2,
+                                        keep_rows=rows)
+    y_ref = wl.oracle_eval(wl.oracle_model(wl.make_model()), sample.numpy())
+    np.testing.assert_allclose(y[:, 0], y_ref, rtol=Y_RTOL, atol=Y_ATOL)

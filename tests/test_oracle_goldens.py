@@ -5,6 +5,8 @@ import copy
 import hashlib
 import json
 import os
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -14,9 +16,39 @@ import golden_io as gio
 from oracle import xpgnn_oracle as orc
 from oracle.mt19937 import MT19937
 
+# The fixtures hold the reference's float32 CPU results, computed on the default code path of the machine that made
+# them.  The WLM fit (Adam on near-cancelling gradients) turns last-bit differences between CPU code paths (FMA
+# contraction, SIMD width of reductions, MKL kernel choice) into weight differences of up to ~4e-7, above the
+# comparison's 1e-7 floor, so on the default path the result depends on the CPU the test runs on.  The comparison
+# therefore runs the oracle in a child process pinned to one code path: MKL's reproducible mode and ATen's scalar
+# kernels on one thread (MKL reproduces results only at a fixed thread count).  On that path the oracle's weights are
+# within the tolerances of the fixtures (worst element at 0.8 of its bound), and the path does not depend on the CPU's
+# instruction set.
+PINNED_CPU_ENV = {"MKL_CBWR": "COMPATIBLE", "ATEN_CPU_CAPABILITY": "default", "OMP_NUM_THREADS": "1",
+                  "MKL_NUM_THREADS": "1"}
+PINNED = all(os.environ.get(k) == v for k, v in PINNED_CPU_ENV.items())
+
+
+@pytest.fixture(scope="module")
+def pinned_child(request):
+    """Outside the pinned environment: runs every case of the comparison once in a pinned child pytest and returns
+    (its exit code, its report with one ``PASSED <node id>`` line per passing case)."""
+    if PINNED:
+        return None
+    cmd = [sys.executable] + (["-s"] if sys.flags.no_user_site else []) + [
+        "-m", "pytest", "-q", "-rA", "-p", "no:cacheprovider",
+        request.node.nodeid + "::test_oracle_explain_matches_reference_golden"]
+    out = subprocess.run(cmd, cwd=str(request.config.rootpath), env=dict(os.environ, **PINNED_CPU_ENV),
+                         capture_output=True, text=True, timeout=900)
+    return out.returncode, out.stdout + out.stderr
+
 
 @pytest.mark.parametrize("name", gio.CASES)
-def test_oracle_explain_matches_reference_golden(name):
+def test_oracle_explain_matches_reference_golden(name, request, pinned_child):
+    if not PINNED:
+        rc, report = pinned_child
+        assert rc == 0 and "PASSED " + request.node.nodeid in report.splitlines(), report[-6000:]
+        return
     case = gio.load_case(name)
     z, meta = case["z"], case["meta"]
     names, pathways, pnames = gio.fresh_inputs(case)
