@@ -665,6 +665,7 @@ int xpgnn_dense_rows(const float* in, int64_t rows, int32_t k, int32_t ld_in, co
                      int32_t act, float* out, int32_t ld_out, int32_t accumulate, int32_t precision, void* stream) {
   XP_REQUIRE(in && w && out && rows >= 0 && rows < (1ll << 31) && k > 0 && n_out > 0, "bad argument");
   XP_REQUIRE(precision >= 0 && precision <= 2, "precision must be 0 (fp32 SIMT), 1 (bf16 tcgen05) or 2 (tf32x3 tcgen05)");
+  if (rows == 0) return 0;  // nothing to transform, in every precision (the tensor-core shape check wants rows > 0)
   DenseArgs d{};
   d.in = in; d.ld_in = ld_in; d.k = k; d.w = w; d.b = b; d.n_out = n_out; d.out = out; d.ld_out = ld_out;
   d.rows_per_s = (int)rows; d.M = rows; d.accumulate = accumulate; d.act_fn = act; d.dst_lo = 0; d.dst_hi = (int)rows;
@@ -678,7 +679,7 @@ int xpgnn_dense_rows(const float* in, int64_t rows, int32_t k, int32_t ld_in, co
 
 int xpgnn_forward(const xpgnn_plan_t* p, const uint32_t* act, int32_t W, int32_t s0, int32_t n_s, float* y, void* workspace,
                   int64_t workspace_bytes, int64_t* stats, void* stream) {
-  XP_REQUIRE(p && act && y && workspace, "null argument");
+  XP_REQUIRE(p && act && workspace && (y || n_s == 0), "null argument");  // an empty range may come with an empty output
   XP_REQUIRE(p->n_layers >= 1 && p->n_nodes > 0 && p->n_query > 0 && p->query, "empty plan");
   XP_REQUIRE(s0 % 32 == 0 && n_s >= 0 && (int64_t)W * 32 >= (int64_t)s0 + n_s, "coalition range outside the bit matrix");
   XP_REQUIRE(p->n_head <= kMaxHead, "head deeper than 8 layers");
