@@ -39,6 +39,11 @@ class Plan(C.Structure):
                 ("out_col", i32), ("prune", i32), ("hop", ptr), ("zero_edge_rule", i32), ("precision", i32)]
 
 
+class FitQuery(C.Structure):
+    _fields_ = [("act_off", i64), ("y_off", i64), ("kern_off", i64), ("w_off", i64), ("n", i32), ("s", i32), ("batch", i32),
+                ("pad_", i32), ("losses", ptr)]
+
+
 CONV_GCN, CONV_SAGE_MEAN = 0, 1
 ACT_NONE, ACT_RELU, ACT_SIGMOID = 0, 1, 2
 
@@ -57,6 +62,10 @@ _SIGNATURES = {
     "xpgnn_pack_mask": (C.c_int, [ptr, i32, i32, ptr, i32, ptr, ptr]),
     "xpgnn_khop_subgraph": (C.c_int, [ptr, i64, i64, i64, i32, ptr, ptr, ptr, ptr, ptr, ptr, ptr]),
     "xpgnn_build_csr": (C.c_int, [ptr, ptr, i64, i64, i32, ptr, ptr, ptr, ptr]),
+    "xpgnn_khop_multi_workspace_bytes": (i64, [i64, i32]),
+    "xpgnn_khop_multi_count": (C.c_int, [ptr, i64, i64, ptr, i32, i32, ptr, i64, ptr, ptr]),
+    "xpgnn_khop_multi_emit": (C.c_int, [ptr, i64, i64, ptr, i32, i32, ptr, i64, ptr, ptr, ptr, i64, ptr, ptr, ptr, ptr, ptr,
+                                        ptr]),
     "xpgnn_forward_workspace_bytes": (i64, [C.POINTER(Plan), i32]),
     "xpgnn_forward": (C.c_int, [C.POINTER(Plan), ptr, i32, i32, i32, ptr, ptr, i64, ptr, ptr]),
     "xpgnn_dense_rows": (C.c_int, [ptr, i64, i32, i32, ptr, ptr, i32, i32, ptr, i32, i32, i32, ptr]),
@@ -64,6 +73,7 @@ _SIGNATURES = {
     "xpgnn_profile_read": (C.c_int, [ptr, ptr]),
     "xpgnn_shap_weights": (C.c_int, [ptr, i32, i32, i32, ptr, ptr, i32, ptr, ptr]),
     "xpgnn_wlm_fit": (C.c_int, [ptr, i32, i32, i32, i32, ptr, ptr, ptr, f64, f64, f64, i32, ptr, ptr]),
+    "xpgnn_wlm_fit_batch": (C.c_int, [ptr, i32, ptr, i64, ptr, ptr, C.POINTER(FitQuery), i32, f64, f64, f64, i32, ptr]),
     "xpgnn_repeat_stats": (C.c_int, [ptr, i32, i32, ptr, ptr, ptr]),
     "xpgnn_community_mean": (C.c_int, [ptr, ptr, ptr, i32, ptr, ptr]),
 }

@@ -43,6 +43,71 @@ def khop_subgraph(edge_index, n_nodes, query, hops):
     return subset, sub_ei, sub_ind, edge_mask[:e].bool(), hop, relabel
 
 
+MAX_QUERIES_PER_KHOP = 64  # one bit per query in the device reach words
+
+
+class MultiKhop:
+    """Block-diagonal union of the k-hop graphs of several queries (``xpgnn_khop_multi_*``).  Block q holds query q's
+    ``subset`` (ascending node ids) in ``subset[node_off[q]:node_off[q+1]]`` with its BFS ``level``s, and its induced
+    edges, in input order and relabelled to union positions, in ``edge_index[:, edge_off[q]:edge_off[q+1]]``.
+    ``sub_ind[q]`` is the query's rank inside its block; ``edge_id`` the input column of each union edge (-1 for the
+    self loop of a query without an induced edge)."""
+
+    def __init__(self, subset, level, sub_ind, edge_index, edge_id, node_off, edge_off):
+        self.subset, self.level, self.sub_ind, self.edge_index, self.edge_id = subset, level, sub_ind, edge_index, edge_id
+        self.node_off, self.edge_off = node_off, edge_off
+
+    def __len__(self):
+        return len(self.node_off) - 1
+
+    def block(self, q):
+        """Query q alone: (subset, local sub_edge_index, sub_ind, level, edge_id) -- what ``khop_subgraph`` gives."""
+        n0, n1, e0, e1 = self.node_off[q], self.node_off[q + 1], self.edge_off[q], self.edge_off[q + 1]
+        return (self.subset[n0:n1], self.edge_index[:, e0:e1] - n0, int(self.sub_ind[q]), self.level[n0:n1],
+                self.edge_id[e0:e1])
+
+
+def khop_subgraph_multi(edge_index, n_nodes, queries, hops):
+    """Device k-hop of up to 64 queries at once (one reach word per node and level, one pass over the edges per hop for
+    all of them).  Every block of the returned ``MultiKhop`` is bit-identical to ``khop_subgraph`` for that query."""
+    lib = _lib.load()
+    dev = require_cuda()
+    queries = [int(q) for q in queries]
+    nq = len(queries)
+    if not 1 <= nq <= MAX_QUERIES_PER_KHOP:
+        raise ValueError("khop_subgraph_multi takes 1..%d queries, got %d" % (MAX_QUERIES_PER_KHOP, nq))
+    if min(queries) < 0 or max(queries) >= n_nodes:
+        raise IndexError("query outside [0, %d)" % n_nodes)
+    ei = edge_index.to(dev, torch.int64).contiguous()
+    e = int(ei.shape[1])
+    qt = torch.tensor(queries, dtype=torch.int64, device=dev)
+    ws_bytes = int(lib.xpgnn_khop_multi_workspace_bytes(int(n_nodes), int(hops)))
+    if ws_bytes < 0:
+        raise ValueError("bad n_nodes / hops")
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    counts = torch.empty(2 * nq + 1, dtype=torch.int64, device=dev)
+    st = _lib.stream_ptr()
+    _lib.check(lib.xpgnn_khop_multi_count(ei.data_ptr(), e, int(n_nodes), qt.data_ptr(), nq, int(hops), ws.data_ptr(),
+                                          ws_bytes, counts.data_ptr(), st))
+    c = counts.tolist()
+    if c[2 * nq]:
+        raise IndexError("edge_index holds %d edge(s) with an endpoint outside [0, %d)" % (c[2 * nq], n_nodes))
+    node_off = np.concatenate([[0], np.cumsum(c[:nq])]).astype(np.int64)
+    edge_off = np.concatenate([[0], np.cumsum(np.maximum(c[nq:2 * nq], 1))]).astype(np.int64)
+    n_u, e_u = int(node_off[-1]), int(edge_off[-1])
+    offs = torch.from_numpy(np.concatenate([node_off, edge_off])).to(dev)
+    subset = torch.empty(n_u, dtype=torch.int64, device=dev)
+    level = torch.empty(n_u, dtype=torch.int8, device=dev)
+    sub_ind = torch.empty(nq, dtype=torch.int64, device=dev)
+    sub_ei = torch.empty((2, e_u), dtype=torch.int64, device=dev)
+    edge_id = torch.empty(e_u, dtype=torch.int64, device=dev)
+    _lib.check(lib.xpgnn_khop_multi_emit(ei.data_ptr(), e, int(n_nodes), qt.data_ptr(), nq, int(hops), ws.data_ptr(), ws_bytes,
+                                         counts.data_ptr(), offs.data_ptr(), offs.data_ptr() + 8 * (nq + 1), e_u,
+                                         subset.data_ptr(), level.data_ptr(), sub_ind.data_ptr(), sub_ei.data_ptr(),
+                                         edge_id.data_ptr(), st))
+    return MultiKhop(subset, level, sub_ind.cpu().tolist(), sub_ei, edge_id, node_off.tolist(), edge_off.tolist())
+
+
 class Data:
     def __init__(self, feat, edge_index):
         self.feat = feat

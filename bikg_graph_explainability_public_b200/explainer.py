@@ -6,21 +6,22 @@ path (k-hop cut, coalition masks, perturbed forward, SHAP weights, surrogate fit
 scores) running in CUDA kernels through ``libxpgnn_b200.so``.  There is no CPU fallback: without
 a CUDA device or without the built library, ``run`` raises.
 """
+import operator
 import random
 
 import numpy as np
 import torch
 
 from . import _lib
-from .data import Data
+from .data import MAX_QUERIES_PER_KHOP, Data, khop_subgraph_multi
 from .engine import GraphSpec, MaskedForward, require_cuda
 from .kernels import shap_weights
 from .lowering import lower
 from .masks import Mask
 from .model import Model
-from .pathways import Pathways, all_str
+from .pathways import CommunityIndex, Pathways, _first_index, all_str
 from .shard import sharded_eval
-from .wlm import LinearRegression, fit_surrogate
+from .wlm import LinearRegression, fit_surrogate, optimizer_assertions
 
 
 def set_seed(seed=100):
@@ -173,6 +174,18 @@ def verify_lowering(arch, feat_dims, node_type_names=None, edge_type_names=None,
         "HeteroConv(sum) with ReLU / Sigmoid, then Linear layers" % "; ".join(worst))
 
 
+_TOO_LARGE = (torch.OutOfMemoryError, torch.AcceleratorError, _lib.XpgnnError)
+
+
+class _GroupTooLarge(Exception):
+    """The union of a group of queries does not fit the device; the group is split."""
+
+
+def _does_not_fit(ex):
+    """A device allocation failed or the engine's workspace does not fit: a smaller group of queries may."""
+    return isinstance(ex, torch.OutOfMemoryError) or "does not fit" in str(ex) or "out of memory" in str(ex)
+
+
 def sync_rng_across_ranks():
     """One process per GPU: every rank replays the coalition stream of the CPU generator, so the generators must agree.
     ``set_seed`` guarantees that only for ``times == 1`` (explainer.py:342); rank 0's state is made authoritative."""
@@ -211,7 +224,8 @@ class Explainer:
     #: products (error ~1e-6 relative, inside the 1e-4 bar); "fp32_exact": exact fp32 FMA transforms (slower, for audits);
     #: "bf16" / "bf16_act": the 2e-2 bar.  verify: compare the
     #: lowered plan with ``arch`` itself on a probe graph before explaining (see ``verify_lowering``).
-    engine_options = dict(prune=True, precision="fp32", verify=True)
+    #: group_size (``run_batch``): queries per k-hop call and per engine, at most 64.
+    engine_options = dict(prune=True, precision="fp32", verify=True, group_size=MAX_QUERIES_PER_KHOP)
 
     def __init__(self, feat, edge_index, arch, params, names, pathways=None, pathway_names=None, element_type=None,
                  problem="node_prediction", node_types=None, edge_types=None):
@@ -439,3 +453,240 @@ class Explainer:
             pathway_df = sub_pathway_class.aggregate(mean, sub_pathway_inds)
         nvtx.range_pop()
         return config_val_df, pathway_df
+
+    # ------------------------------------------------------------------ many queries
+    def run_batch(self, elements, times=1):
+        """Explain several query nodes: returns ``[Explainer(<same constructor args>).run(e, times) for e in elements]``,
+        run from the same global CPU generator state, which it also leaves as that loop does.
+
+        The query-independent work runs once: flattening, the plan check (``verify_lowering``), the name -> index map and
+        the community members' ids.  The queries' computational graphs are cut together (``khop_subgraph_multi``), laid
+        side by side as one block-diagonal graph and evaluated by ONE engine call over all their coalitions; their
+        surrogates are fitted together (``xpgnn_wlm_fit_batch``).  Queries go in groups of at most ``group_size`` (64),
+        in input order; a group whose engine does not fit the device is split.
+
+        Node problems on homogeneous graphs and on dict graphs with one node type.  Raises ``NotImplementedError`` for
+        graph and edge problems, graphs with two or more node types and caller-provided node / edge type vectors.
+        With ``options["keep_last"]`` the intermediates ``run`` keeps in ``_last`` go to the list ``_last_batch``;
+        ``last_stats`` is a list with one dict per query."""
+        import gc
+
+        gc_was_enabled = gc.isenabled()
+        gc.disable()
+        try:
+            return self._run_batch(list(elements), times)
+        finally:
+            if gc_was_enabled:
+                gc.enable()
+
+    def _run_batch(self, elements, times):
+        dev = require_cuda()
+        _lib.load()
+        if "edge" in self.problem:
+            raise NotImplementedError("edge problems: the reference path is not runnable (data.py:359, masks.py:294); not built")
+        if "graph" in self.problem:
+            raise NotImplementedError("run_batch explains node problems; a graph problem reads the whole graph for every "
+                                      "element, there is no computational graph to batch: use run")
+        if self.node_types is not None or self.edge_types is not None:
+            raise NotImplementedError("run_batch does not batch caller-provided node / edge type vectors (the 5-argument "
+                                      "forward): use run")
+        if isinstance(self.feat, dict) and len(self.feat) >= 2:
+            raise NotImplementedError("run_batch does not batch graphs with two or more node types: their zero-edge rule "
+                                      "(model.py:213-215) applies per coalition of one query's graph, the engine would "
+                                      "apply it over the whole union; use run")
+        nvtx = torch.cuda.nvtx
+        nvtx.range_push("xpgnn:run_batch:flatten")
+        raw = Data(self.feat, self.edge_index)
+        if self.pathways is not None:
+            raw_pathways = Pathways(self.pathways, self.pathway_names)
+        (ntn, etn, self.feat, self.edge_index, node_types, edge_types, nptr, eptr, pads) = raw.preprocess_hetero_graph()
+        self.names, _ = raw.hetero2homo_names(self.names)
+        if self.pathways is not None:
+            self.pathways, self.pathway_names, _ptypes = raw_pathways.hetero2homo(self.problem, nptr, eptr)
+        first = _first_index(self.names) if all_str(self.names) else None
+        inds = []
+        for e in elements:
+            if first is not None and type(e) is str:
+                assert e in first, "Element name '{}' is not present in the graph".format(e)
+                inds.append(first[e])
+            else:
+                inds.append(self.extract_index(e, self.names))
+        nvtx.range_pop()
+        nvtx.range_push("xpgnn:run_batch:communities")
+        cindex = None
+        if self.pathways is not None:
+            cindex = CommunityIndex(self.pathways, self.pathway_names, self.names, first)
+        nvtx.range_pop()
+        nvtx.range_push("xpgnn:run_batch:engine_build")
+        opts = dict(type(self).engine_options)
+        opts.update(getattr(self, "options", {}))
+        group = max(1, min(int(opts.get("group_size", MAX_QUERIES_PER_KHOP)), MAX_QUERIES_PER_KHOP))
+        out_type = self.element_type if isinstance(self.element_type, str) else None
+        self.arch.eval()
+        plan = None
+        self.lowering_status = "not checked"
+        if opts.get("verify", True):
+            fd = int(self.feat.shape[1]) if ntn is None else {t: int(self.feat.shape[1]) - int(pads[i]) for i, t in enumerate(ntn)}
+            plan, self.lowering_status = verify_lowering(self.arch, fd, ntn, etn, out_type)
+        nvtx.range_pop()
+        nvtx.range_push("xpgnn:run_batch:khop")
+        feat = self.feat.to(dev)
+        edge_index = self.edge_index.to(dev)
+        n_hops = Model(self.arch).get_hops(len(etn) if etn is not None else 0) + 1  # data.py:328: one more hop
+        del self.feat, self.edge_index  # explainer.py:476: the object is single use
+        nvtx.range_pop()
+        ctx = dict(feat=feat, node_types=None if node_types is None else node_types.to(dev),
+                   edge_types=None if edge_types is None else edge_types.to(dev), ntn=ntn, etn=etn, pads=pads,
+                   out_type=out_type, plan=plan, opts=opts, times=times, cindex=cindex)
+        self.last_stats = []
+        if opts.get("keep_last", False):
+            self._last_batch = []
+        results = []
+        for g0 in range(0, len(inds), group):
+            results += self._explain_group(edge_index, inds[g0:g0 + group], n_hops, ctx)
+        return results
+
+    def _explain_group(self, edge_index, inds, n_hops, ctx):
+        """Cut the computational graphs of ``inds`` together and explain them; halves the group when the union does not
+        fit the device."""
+        nvtx = torch.cuda.nvtx
+        nvtx.range_push("xpgnn:run_batch:khop")
+        try:
+            mk = khop_subgraph_multi(edge_index, int(ctx["feat"].shape[0]), inds, n_hops)
+        except _TOO_LARGE as ex:
+            if not _does_not_fit(ex) or len(inds) == 1:
+                raise
+            mk = None
+        nvtx.range_pop()
+        if mk is not None:
+            try:
+                return self._explain_union(mk, ctx)
+            except _GroupTooLarge:  # raised before any coalition of the group is drawn: halving keeps the draw order
+                pass
+        mk = None
+        torch.cuda.empty_cache()  # the library's stream-ordered scratch does not come from torch's cache
+        h = len(inds) // 2
+        return self._explain_group(edge_index, inds[:h], n_hops, ctx) + self._explain_group(edge_index, inds[h:], n_hops, ctx)
+
+    def _explain_union(self, mk, ctx):
+        """Explain the queries of one block-diagonal union (``MultiKhop``); splits it when its engine does not fit."""
+        nvtx = torch.cuda.nvtx
+        opts, times, nq = ctx["opts"], ctx["times"], len(mk)
+        nvtx.range_push("xpgnn:run_batch:engine_build")
+        queries = [mk.node_off[q] + mk.sub_ind[q] for q in range(nq)]
+        try:
+            sub_feat = ctx["feat"][mk.subset]
+            sub_nt = None if ctx["node_types"] is None else ctx["node_types"][mk.subset]
+            sub_et = None
+            if ctx["edge_types"] is not None:  # a self loop of the per-query rule (edge_id -1) belongs to no relation
+                sub_et = torch.where(mk.edge_id >= 0, ctx["edge_types"][mk.edge_id.clamp(min=0)].to(torch.int64), -1)
+            engine = build_engine(sub_feat, mk.edge_index, self.arch, 0, sub_nt, sub_et, ctx["ntn"], ctx["etn"], ctx["pads"],
+                                  out_type=ctx["out_type"], hop=mk.level, prune=opts["prune"], precision=opts["precision"],
+                                  model=ctx["plan"], queries=queries)
+        except _TOO_LARGE as ex:
+            nvtx.range_pop()
+            if not _does_not_fit(ex) or nq == 1:
+                raise
+            raise _GroupTooLarge() from None
+        nvtx.range_pop()
+        nvtx.range_push("xpgnn:run_batch:communities")
+        subset_host = mk.subset.cpu()
+        idx_all = subset_host.tolist()
+        names = self.names
+        str_names = all_str(names)
+        per_q = []
+        for q in range(nq):
+            n0, n1 = mk.node_off[q], mk.node_off[q + 1]
+            idx = idx_all[n0:n1]
+            if str_names:  # == Data.comp_graph's names[subset]
+                sub_names = list(operator.itemgetter(*idx)(names)) if len(idx) > 1 else [names[i] for i in idx]
+            else:
+                sub_names = np.array(names, dtype=str)[idx].tolist()
+            com_inds = com_names = None
+            if ctx["cindex"] is not None:
+                com_inds, com_names = ctx["cindex"].resolve(subset_host[n0:n1].numpy())
+                if not com_inds:
+                    raise IndexError("list index out of range")  # explainer.py:467: no community reaches the graph
+            per_q.append(dict(n=n1 - n0, sub_names=sub_names, com_inds=com_inds, com_names=com_names))
+        nvtx.range_pop()
+        # ---- every query's coalitions, in input order, with the draw sequence of run (masks -> surrogate init -> the
+        # DataLoader seed draw, per repeat; set_seed per query when times == 1) ----
+        nvtx.range_push("xpgnn:run_batch:masks")
+        sync_rng_across_ranks()
+        for q, pq in enumerate(per_q):
+            if times == 1:
+                set_seed(self.params["seed"])
+            n0, n1 = mk.node_off[q], mk.node_off[q + 1]
+            sub_feat_q = sub_feat[n0:n1]
+            sets = []
+            for _ in range(times):
+                coalitions, _rows = Mask(sub_feat_q, None, pq["com_inds"], self.params, self.problem).mask_generator()
+                wlrm = LinearRegression(pq["n"])
+                torch.empty((), dtype=torch.int64).random_()
+                sets.append((coalitions, wlrm.layer.weight.detach().reshape(-1)))
+            pq["sets"] = sets
+            if times == 1:
+                pq["act"], pq["n_all"] = sets[0][0].act, sets[0][0].n_coalitions
+            else:
+                pq["act"] = torch.cat([c.act for c, _ in sets], dim=1)
+                pq["n_all"] = 32 * int(pq["act"].shape[1])
+        w_max = max(int(pq["act"].shape[1]) for pq in per_q)
+        act = torch.zeros((int(mk.node_off[-1]), w_max), dtype=torch.int32, device=engine.device)
+        for q, pq in enumerate(per_q):  # words >= W_q stay zero: every node of the block is off there
+            act[mk.node_off[q]:mk.node_off[q + 1], :pq["act"].shape[1]] = pq["act"]
+        n_all = max(pq["n_all"] for pq in per_q)
+        check_ranks_agree(act)
+        nvtx.range_pop()
+        nvtx.range_push("xpgnn:run_batch:masked_forward")
+        y_all = sharded_eval(engine, act, n_all).contiguous()  # (n_all, nq): column q = query q
+        nvtx.range_pop()
+        nvtx.range_push("xpgnn:run_batch:fit")
+        lib = _lib.load()
+        lr = optimizer_assertions(self.params)
+        descs, kerns, w0s, off = [], [], [], 0
+        for q, pq in enumerate(per_q):
+            word0 = 0
+            pq["w_off"], pq["kern"] = [], []
+            for coalitions, w0 in pq["sets"]:
+                kern = shap_weights(coalitions.popcount, pq["n"], coalitions.batch_size)
+                d = _lib.FitQuery()
+                d.act_off, d.y_off = mk.node_off[q] * w_max + word0, 32 * word0 * nq + q
+                d.kern_off, d.w_off = sum(int(k.numel()) for k in kerns), off
+                d.n, d.s, d.batch, d.losses = pq["n"], coalitions.n_coalitions, coalitions.batch_size, None
+                descs.append(d)
+                kerns.append(kern.to(torch.float64))
+                w0s.append(w0.to(engine.device, torch.float32))
+                pq["w_off"].append(off)
+                pq["kern"].append(kern)
+                off += pq["n"]
+                word0 += coalitions.words
+        kern_all = torch.cat(kerns).contiguous()
+        w_all = torch.cat(w0s).contiguous()
+        arr = (_lib.FitQuery * len(descs))(*descs)
+        _lib.check(lib.xpgnn_wlm_fit_batch(act.data_ptr(), w_max, y_all.data_ptr(), nq, kern_all.data_ptr(), w_all.data_ptr(),
+                                           arr, len(descs), float(lr), float(self.params["l1_lambda"]), 1e-2,
+                                           int(bool(engine.broadcast_y)), _lib.stream_ptr()))
+        nvtx.range_pop()
+        nvtx.range_push("xpgnn:run_batch:aggregate")
+        out = []
+        for q, pq in enumerate(per_q):
+            ws = [w_all[o:o + pq["n"]] for o in pq["w_off"]]
+            mean, std = self.weight_stacking(ws)
+            config_val_df = Data.config_val_dataframe(mean, std, pq["sub_names"])
+            pathway_df = None
+            if pq["com_inds"] is not None:
+                pathway_df = Pathways(pq["com_inds"], pq["com_names"]).aggregate(mean, pq["com_inds"])
+            out.append((config_val_df, pathway_df))
+            coalitions, w0 = pq["sets"][-1]
+            word0 = sum(c.words for c, _ in pq["sets"][:-1])
+            self.last_stats.append(dict(n_sub=pq["n"], e_sub=mk.edge_off[q + 1] - mk.edge_off[q],
+                                        coalitions=coalitions.n_coalitions, batch_size=coalitions.batch_size,
+                                        tile_coalitions=engine.tile_coalitions, repeats_per_engine_call=times,
+                                        queries_per_engine_call=nq, lowering=self.lowering_status))
+            if opts.get("keep_last", False):
+                subset, sub_ei, sub_ind, _lev, _eid = mk.block(q)
+                self._last_batch.append(dict(coalitions=coalitions, y=y_all[32 * word0: 32 * word0 + coalitions.n_coalitions, q],
+                                             kernel=pq["kern"][-1], w0=w0, subset_names=pq["sub_names"],
+                                             sub_edge_index=sub_ei, sub_ind=sub_ind))
+        nvtx.range_pop()
+        return out

@@ -38,6 +38,65 @@ def _first_index(names):
     return dict(zip(reversed(names), range(n - 1, -1, -1)))
 
 
+class CommunityIndex:
+    """Communities resolved once against the global node ids, then per computational graph by id (``Explainer.run_batch``).
+
+    Every id a member name has is kept (names may repeat).  ``resolve(subset)`` gives, for the graph whose ascending
+    global node ids are ``subset``, exactly what ``Pathways(...).resolve_indices(names[subset])`` gives: a name's index is
+    its first occurrence among the graph's names, i.e. the smallest subgraph rank among its ids; communities without a
+    member in the graph are dropped; index lists ascending."""
+
+    def __init__(self, communities, community_names, names, first=None):
+        names = _as_str(names)
+        if first is None:
+            first = _first_index(names)
+        extra = {}  # name -> its ids after the first (repeated names)
+        if len(first) < len(names):
+            firsts = np.fromiter(map(first.__getitem__, names), dtype=np.int64, count=len(names))
+            for i in np.nonzero(firsts != np.arange(len(names)))[0].tolist():
+                extra.setdefault(names[i], []).append(i)
+        com, key, gid = [], [], []
+        for c, community in enumerate(communities):
+            members = _as_str(community)
+            ids = np.fromiter(map(first.get, members, itertools.repeat(-1)), dtype=np.int64, count=len(members))
+            ids = ids[ids >= 0]
+            com.append(np.full(ids.size, c, dtype=np.int64))
+            key.append(ids)
+            gid.append(ids)
+            if extra:
+                for m in set(members) & extra.keys():
+                    more = np.asarray(extra[m], dtype=np.int64)
+                    com.append(np.full(more.size, c, dtype=np.int64))
+                    key.append(np.full(more.size, first[m], dtype=np.int64))
+                    gid.append(more)
+        cat = lambda parts: np.concatenate(parts) if parts else np.zeros(0, dtype=np.int64)  # noqa: E731
+        self.com, self.key, self.gid = cat(com), cat(key), cat(gid)
+        self.community_names = np.arange(len(communities)).tolist() if community_names is None else list(community_names)
+
+    def resolve(self, subset):
+        """``subset``: ascending global node ids of one computational graph.  Returns (index lists, community names)."""
+        subset = np.asarray(subset, dtype=np.int64)
+        if subset.size == 0 or self.gid.size == 0:
+            return [], []
+        pos = np.searchsorted(subset, self.gid)
+        present = subset[np.minimum(pos, subset.size - 1)] == self.gid
+        c, k, r = self.com[present], self.key[present], pos[present]
+        o = np.lexsort((r, k, c))  # per (community, name): the smallest rank
+        c, k, r = c[o], k[o], r[o]
+        head = np.ones(c.size, dtype=bool)
+        head[1:] = (c[1:] != c[:-1]) | (k[1:] != k[:-1])
+        c, r = c[head], r[head]
+        o = np.lexsort((r, c))  # per community: distinct ranks, ascending
+        c, r = c[o], r[o]
+        head = np.ones(c.size, dtype=bool)
+        head[1:] = (c[1:] != c[:-1]) | (r[1:] != r[:-1])
+        c, r = c[head], r[head]
+        if c.size == 0:
+            return [], []
+        kept, starts = np.unique(c, return_index=True)
+        return [part.tolist() for part in np.split(r, starts[1:])], [self.community_names[i] for i in kept.tolist()]
+
+
 class Pathways:
     def __init__(self, communities, community_names, community_types=None):
         self.communities = communities

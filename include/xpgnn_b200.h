@@ -131,6 +131,30 @@ int xpgnn_khop_subgraph(const int64_t* edge_index, int64_t E, int64_t N, int64_t
 int xpgnn_build_csr(const int64_t* src, const int64_t* dst, int64_t E, int64_t N, int32_t drop_self_loops,
                     int32_t* rowptr, int32_t* col, int64_t* n_kept, void* stream);
 
+/* Multi-query k-hop: the computational graphs of Q <= 64 queries (repeats allowed) in the passes one
+ * query needs.  One uint64 reach word per node and level (bit q = reached from queries[q] at that
+ * level, PyG's re-expansion of the whole previous level), so the workspace is
+ * xpgnn_khop_multi_workspace_bytes(N, hops) = 8 N (hops + 1) plus a few KB, independent of E and Q.
+ * Two calls share the caller-held workspace:
+ *   count: counts int64 [2Q + 1] = {N_q for every q, E_q for every q (before the self-loop rule),
+ *          number of edges with an endpoint outside [0, N)};
+ *   emit:  node_off / edge_off int64 [Q + 1] are the caller's exclusive prefix sums of N_q and of
+ *          max(E_q, 1), in device memory; the union is written block by block:
+ *          subset int64 [node_off[Q]] (each query's node ids ascending), level int8 [node_off[Q]]
+ *          (first level the node was reached at from its query), sub_ind int64 [Q] (rank of the query
+ *          inside its own block), sub_edge_index int64 [2][edge_off[Q]] (row stride edge_off[Q]; each
+ *          query's induced edges in original order, relabelled to union positions, i.e. node_off[q]
+ *          added) and edge_id int64 [edge_off[Q]] (optional: the input column of each union edge).
+ *          A query with no induced edge gets one self loop on itself (edge_id -1), as
+ *          xpgnn_khop_subgraph does.  Every block equals what xpgnn_khop_subgraph gives for that query. */
+int64_t xpgnn_khop_multi_workspace_bytes(int64_t N, int32_t hops);
+int xpgnn_khop_multi_count(const int64_t* edge_index, int64_t E, int64_t N, const int64_t* queries, int32_t Q,
+                           int32_t hops, void* workspace, int64_t workspace_bytes, int64_t* counts, void* stream);
+int xpgnn_khop_multi_emit(const int64_t* edge_index, int64_t E, int64_t N, const int64_t* queries, int32_t Q,
+                          int32_t hops, const void* workspace, int64_t workspace_bytes, const int64_t* counts,
+                          const int64_t* node_off, const int64_t* edge_off, int64_t n_union_edges, int64_t* subset,
+                          int8_t* level, int64_t* sub_ind, int64_t* sub_edge_index, int64_t* edge_id, void* stream);
+
 /* ------------------------------------------------------------------------------------------
  * a5/a6/a7  coalition-batched masked message passing
  * replaces: Data.perturbator / build_edge_mask / perturb_node / concat_features
@@ -237,6 +261,23 @@ int xpgnn_shap_weights(const int32_t* popcount, int32_t S, int32_t M, int32_t ba
 int xpgnn_wlm_fit(const uint32_t* act, int32_t W, int32_t N, int32_t S, int32_t batch, const float* y,
                   const double* kern, float* w, double lr, double l1_lambda, double weight_decay,
                   int32_t broadcast_y, double* losses, void* stream);
+
+/* One surrogate of xpgnn_wlm_fit_batch: its coalition bits start at act[act_off] (row stride W of the
+ * call), its predictions at y[y_off] (row stride ldy of the call), its kernel weights at kern[kern_off],
+ * its weights at w[w_off] (N entries, initial in, fitted out); losses (optional) double [ceil(S / batch)]. */
+typedef struct {
+  int64_t act_off, y_off, kern_off, w_off;
+  int32_t n, s, batch, pad_;
+  double* losses;
+} xpgnn_fit_query_t;
+
+/* Q independent xpgnn_wlm_fit problems in one launch sequence: three launches per step index for the
+ * whole batch; a surrogate with fewer steps drops out of later launches.  Every surrogate's weights
+ * and losses are bit-identical to xpgnn_wlm_fit on the same inputs.  The hyper-parameters and
+ * broadcast_y are shared. */
+int xpgnn_wlm_fit_batch(const uint32_t* act, int32_t W, const float* y, int64_t ldy, const double* kern, float* w,
+                        const xpgnn_fit_query_t* queries_host, int32_t Q, double lr, double l1_lambda,
+                        double weight_decay, int32_t broadcast_y, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * a10  aggregation
