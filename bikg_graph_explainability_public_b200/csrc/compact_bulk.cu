@@ -41,6 +41,7 @@
 #include <cstring>
 #include <map>
 #include <mutex>
+#include <tuple>
 #include <utility>
 
 #include "compact_internal.cuh"
@@ -483,37 +484,6 @@ __global__ void __launch_bounds__(32 * (1 + P + C), MINB) cspmm_bulk_kernel(cons
   }
 }
 
-// 2-D tensor map over the chunk-major operand buffer seen as [rows][32 floats] (box = one 128-byte row: the gather4 form
-// loads four of them per instruction).  Encoding goes through the driver entry point (no link dependency on libcuda).
-typedef CUresult (*BgEncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
-                               const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-int bg_tensor_map(const float* base, uint64_t rows, CUtensorMap* out) {
-  static std::mutex mu;
-  static std::map<std::pair<const void*, uint64_t>, CUtensorMap> cache;
-  static BgEncodeFn encode = nullptr;
-  std::lock_guard<std::mutex> lock(mu);
-  auto it = cache.find({base, rows});
-  if (it != cache.end()) { *out = it->second; return 0; }
-  if (!encode) {
-    cudaDriverEntryPointQueryResult qres;
-    XP_CHECK(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", (void**)&encode, cudaEnableDefault, &qres));
-    XP_REQUIRE(encode != nullptr, "cuTensorMapEncodeTiled is not available");
-  }
-  CUtensorMap m;
-  memset(&m, 0, sizeof m);
-  const cuuint64_t dims[2] = {32, rows};
-  const cuuint64_t strides[1] = {128};
-  const cuuint32_t box[2] = {32, 1};
-  const cuuint32_t estr[2] = {1, 1};
-  const CUresult r = encode(&m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                            CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  XP_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled failed");
-  if (cache.size() > 64) cache.clear();
-  cache[{base, rows}] = m;
-  *out = m;
-  return 0;
-}
-
 template <int NS, int MODE, int P, int C, int MINB>
 int bg_launch(const CspmmArgs& a, const CUtensorMap& tmap, cudaStream_t st, int variant) {
   void (*k)(const CspmmArgs, const CUtensorMap) = cspmm_bulk_kernel<NS, MODE, P, C, MINB>;
@@ -539,6 +509,36 @@ int bg_launch(const CspmmArgs& a, const CUtensorMap& tmap, cudaStream_t st, int 
 
 }  // namespace
 
+// Encoding goes through the driver entry point (no link dependency on libcuda).
+typedef CUresult (*BgEncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
+                               const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+int rows128_tensor_map(const float* base, uint64_t rows, bool swizzle128, CUtensorMap* out) {
+  static std::mutex mu;
+  static std::map<std::tuple<const void*, uint64_t, bool>, CUtensorMap> cache;
+  static BgEncodeFn encode = nullptr;
+  std::lock_guard<std::mutex> lock(mu);
+  auto it = cache.find({base, rows, swizzle128});
+  if (it != cache.end()) { *out = it->second; return 0; }
+  if (!encode) {
+    cudaDriverEntryPointQueryResult qres;
+    XP_CHECK(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", (void**)&encode, cudaEnableDefault, &qres));
+    XP_REQUIRE(encode != nullptr, "cuTensorMapEncodeTiled is not available");
+  }
+  CUtensorMap m;
+  memset(&m, 0, sizeof m);
+  const cuuint64_t dims[2] = {32, rows};
+  const cuuint64_t strides[1] = {128};
+  const cuuint32_t box[2] = {32, 1};
+  const cuuint32_t estr[2] = {1, 1};
+  const CUresult r = encode(&m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                            swizzle128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  XP_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled failed");
+  if (cache.size() > 64) cache.clear();
+  cache[{base, rows, swizzle128}] = m;
+  *out = m;
+  return 0;
+}
+
 int launch_cspmm_bulk(const CspmmArgs& a, int variant, cudaStream_t st) {
   // variant = 100 * mode + ring stages (16 | 32); mode 0 bulk copies | 1 cp.async.cg | 2 cp.async.ca | 3 TMA gather4 |
   // 4 TMA gather4, the small configuration that runs next to cspmm_seg_kernel (2 producer + 4 consumer warps, 16 stages)
@@ -549,7 +549,7 @@ int launch_cspmm_bulk(const CspmmArgs& a, int variant, cudaStream_t st) {
     XP_REQUIRE(a.in_s_stride % 32 == 0 && a.in_chunk_stride % 32 == 0, "gather4: operand strides must be whole 128-byte rows");
     const uint64_t rows = (uint64_t)((int64_t)(a.nb - 1) * a.in_s_stride + (int64_t)(a.n_chunks - 1) * a.in_chunk_stride) / 32 + (uint64_t)a.N;
     XP_REQUIRE(rows < (1ull << 31), "gather4: row index does not fit 31 bits");
-    if (bg_tensor_map(a.in, rows, &tmap)) return 1;
+    if (rows128_tensor_map(a.in, rows, false, &tmap)) return 1;
   }
   if (mode == 4) return bg_launch<16, 3, 2, 4, 2>(a, tmap, st, variant);
   if (ns >= 32) {

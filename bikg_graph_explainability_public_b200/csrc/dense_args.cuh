@@ -1,5 +1,7 @@
 // Arguments of the dense row transform, shared by the SIMT (engine.cu) and tensor-core (dense_tc.cu) paths.
 #pragma once
+#include <cuda.h>
+
 #include "common.cuh"
 
 namespace xpgnn {
@@ -88,6 +90,9 @@ __device__ __forceinline__ int64_t dense_out_off(const DenseArgs& a, int n) {
 
 enum { DENSE_SIMT = 0, DENSE_TC_BF16 = 1, DENSE_TC_TF32X3 = 2 };
 bool dense_tc_eligible(const DenseArgs& d, int mode /*0 tf32x3, 1 bf16*/);
+// 2-D tensor map over a float buffer seen as [rows][32 floats] with a 128-byte pitch, box = one row (the gather4 form loads
+// four of them per instruction); swizzle128: land the rows in the K-major SWIZZLE_128B layout.  Cached per (base, rows, swizzle).
+int rows128_tensor_map(const float* base, uint64_t rows, bool swizzle128, CUtensorMap* out);
 int launch_dense_tc(const DenseArgs& d, int mode, cudaStream_t st);
 
 }  // namespace xpgnn

@@ -7,14 +7,19 @@
 //            (hi*hi + lo*hi + hi*lo).  Error ~2^-20 relative: keeps the fp32 parity bar (1e-4).
 //   BF16   : operands rounded to bf16, one MMA per K step (the "bf16 transforms" mode, 2e-2 bar).
 // Operands are staged in shared memory in the canonical no-swizzle K-major core-matrix layout
-// (8 rows x 16 bytes per core matrix) by plain vectorised loads -- the A operand is produced by the
-// masked SpMM in a fused pipeline, so TMA tensor maps would not apply to it.  One elected thread
-// issues the MMAs; completion is tracked with tcgen05.commit -> mbarrier; the epilogue reads the
-// accumulator tile with tcgen05.ld (32 lanes x 32 columns per warp instruction).
+// (8 rows x 16 bytes per core matrix) by plain vectorised loads -- except the A operand of TF32x3 transforms whose
+// input is chunk-major with 32-float chunks and whose rows come from the tile table (the layer >= 1 transforms of the
+// compact paths): there each 128-row x 32-float stage is gathered by TMA (gather4, 4 rows of 128 bytes per
+// instruction) into the K-major SWIZZLE_128B layout, and the tensor core reads the landed fp32 rows directly as the hi
+// operand -- kind::tf32 uses only the top 19 bits of an element, which is exactly the truncated hi of the split.
+// Converter warps write lo = a - hi next to it.  One elected thread issues the MMAs; completion is tracked with
+// tcgen05.commit -> mbarrier; the epilogue reads the accumulator tile with tcgen05.ld (32 lanes x 32 columns per warp
+// instruction).
 #include <cuda_bf16.h>
 
 #include <algorithm>
 #include <cstdlib>
+#include <cstring>
 
 #include "common.cuh"
 #include "dense_args.cuh"
@@ -137,6 +142,27 @@ __device__ __forceinline__ uint64_t smem_desc(uint32_t saddr, uint32_t lbo_bytes
   d |= (uint64_t)1 << 46;  // descriptor version (Blackwell)
   return d;                // base offset 0, lbo mode 0, layout type 0 (SWIZZLE_NONE)
 }
+// K-major SWIZZLE_128B: rows of 128 bytes, 8-row atoms of 1024 bytes (SBO), 16-byte column c of row r stored at column
+// c ^ (r & 7) -- the layout TMA writes with CU_TENSOR_MAP_SWIZZLE_128B.  The atom must be 1024-byte aligned (base offset
+// 0); a K step inside the atom advances the start address by its byte offset (the swizzle applies to the final address).
+__device__ __forceinline__ uint64_t smem_desc_sw128(uint32_t saddr) {
+  uint64_t d = 0;
+  d |= (uint64_t)((saddr >> 4) & 0x3fffu);
+  d |= (uint64_t)1 << 16;               // LBO: unused for K-major swizzled operands one atom wide
+  d |= (uint64_t)(1024 >> 4) << 32;     // SBO
+  d |= (uint64_t)1 << 46;
+  d |= (uint64_t)2 << 61;               // layout type SWIZZLE_128B
+  return d;
+}
+__device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes) {
+  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
+}
+// TMA gather4: rows r0 .. r3 (128 bytes each) of the 2-D tensor map -> 4 consecutive 128-byte rows at smem_dst
+__device__ __forceinline__ void tma_gather4(uint32_t smem_dst, const CUtensorMap* tmap, int r0, int r1, int r2, int r3, uint64_t* bar) {
+  asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.tile::gather4.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6, %7}], [%2];" ::"r"(smem_dst),
+               "l"(tmap), "r"(smem_u32(bar)), "r"(0), "r"(r0), "r"(r1), "r"(r2), "r"(r3)
+               : "memory");
+}
 __host__ __device__ constexpr uint32_t make_idesc(int kind_fmt /*1 bf16, 2 tf32*/, int M, int N) {
   return (1u << 4) | ((uint32_t)kind_fmt << 7) | ((uint32_t)kind_fmt << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
@@ -148,6 +174,14 @@ constexpr int LOADER_GROUPS = 3;  // chunks in flight per SM
 constexpr int GROUP_WARPS = 4;
 constexpr int LOADER_WARPS = GROUP_WARPS * LOADER_GROUPS;
 constexpr int TC_THREADS = 32 * (EPI_WARPS + LOADER_WARPS + 1);  // warps 0-7 epilogue, 8-19 loaders / converters, 20 MMA issue
+// gather4 form (G4): warps 0-7 epilogue, 8-9 converters (one 16 KB lo stage per item), 10 MMA issue, 11-14 TMA producers
+// (15 warps: up to 128 registers a thread)
+constexpr int G4_CONV_WARPS = 2;
+constexpr int G4_PROD_WARPS = 4;
+constexpr int G4_THREADS = 32 * (EPI_WARPS + G4_CONV_WARPS + 1 + G4_PROD_WARPS);
+constexpr int G4_LO = 2;          // lo stages (held from conversion to MMA completion)
+constexpr int G4_MAX_HI = 4;      // landed hi stages (held from the TMA issue to MMA completion: more of them)
+constexpr int G4_PART = 128 * 128;  // bytes of one 128-row x 32-float stage part
 constexpr int MAX_DONE = 12;      // lcm(stages <= 4, LOADER_GROUPS)
 constexpr int KC = 32;           // K elements per stage
 constexpr int MAX_STAGES = 4;
@@ -236,8 +270,17 @@ __device__ __noinline__ const float* resolve_in_row(const float* in, int64_t in_
 //                       buffers in TMEM, commits to "stage empty" and, after the last chunk, "accumulator full";
 //   epilogue (4 warps): waits "accumulator full", tcgen05.ld, bias / accumulate / activation / row scale,
 //                       stores, then "accumulator empty".  It overlaps the next tile's loads and MMAs.
-template <int MODE>
-__global__ void __launch_bounds__(TC_THREADS, 1) dense_tc_kernel(const DenseArgs a, int n_pad, uint32_t tmem_cols, int n_stages, unsigned long long* dbg) {
+// G4 (MODE 0, chunk-major 32-float input, tile-table rows): the loaders are replaced by
+//   TMA producers (4 warps): per item 32 gather4 (8 per warp, 4 tile rows each) into a landed "hi" stage, counted in
+//                       bytes on its mbarrier; n_stages hi stages, refilled when the MMAs of the item that used them are done;
+//   converters (2 warps): read the landed stage, write lo = a - (a & 0xffffe000) to one of G4_LO lo stages (same
+//                       swizzled layout, so element positions match one to one), arrive "stage full".
+template <int MODE, bool G4>
+__global__ void __launch_bounds__(G4 ? G4_THREADS : TC_THREADS, 1)
+    dense_tc_kernel(const DenseArgs a, int n_pad, uint32_t tmem_cols, int n_stages, unsigned long long* dbg, const __grid_constant__ CUtensorMap tmap) {
+  static_assert(!G4 || MODE == 0, "the gather4 path feeds the TF32x3 MMAs");
+  constexpr int NT = G4 ? G4_THREADS : TC_THREADS;
+  constexpr int MMA_WARP = EPI_WARPS + (G4 ? G4_CONV_WARPS : LOADER_WARPS);
   using Cfg = TcCfg<MODE>;
   extern __shared__ __align__(128) uint8_t smem[];
   __shared__ uint64_t bar_full[MAX_STAGES];
@@ -254,13 +297,19 @@ __global__ void __launch_bounds__(TC_THREADS, 1) dense_tc_kernel(const DenseArgs
   const int kb16 = K * Cfg::ELT / 16;                 // 16-byte columns of a full-K row
   const uint32_t b_part_bytes = (uint32_t)n_pad * K * Cfg::ELT;
   uint8_t* sB = smem;                                      // [PARTS][n_pad x K]
-  uint8_t* sA = smem + (size_t)b_part_bytes * Cfg::PARTS;  // [n_stages][PARTS][TM x KC]
+  uint8_t* sA = smem + (size_t)b_part_bytes * Cfg::PARTS;  // [n_stages][PARTS][TM x KC] | G4: [n_stages] hi, [G4_LO] lo
+  if (G4) sA = smem + ((smem_u32(sA) + 1023u) & ~1023u) - smem_u32(smem);  // SWIZZLE_128B atoms: 1024-byte aligned
+  // G4 barriers: bar_full[G4_LO] = lo stage written (converters), hi_full = hi stage landed (TMA bytes),
+  // hi_empty / lo_empty = the MMAs reading the stage are done (tcgen05.commit)
+  uint64_t* hi_full = bar_done;
+  uint64_t* hi_empty = bar_done + G4_MAX_HI;
+  uint64_t* lo_empty = bar_done + 2 * G4_MAX_HI;
 
   if (warp == 0) tmem_alloc(&tmem_base_sh, tmem_cols);
   if (tid < 256) s_bias[tid] = (a.b && tid < a.n_out) ? a.b[tid] : 0.0f;
   if (tid == 0) {
-    for (int s = 0; s < MAX_STAGES; ++s) mbar_init(&bar_full[s], 32 * GROUP_WARPS);
-    for (int s = 0; s < MAX_DONE; ++s) mbar_init(&bar_done[s], 1);
+    for (int s = 0; s < MAX_STAGES; ++s) mbar_init(&bar_full[s], 32 * (G4 ? G4_CONV_WARPS : GROUP_WARPS));
+    for (int s = 0; s < MAX_DONE; ++s) mbar_init(&bar_done[s], (G4 && s < G4_MAX_HI) ? G4_PROD_WARPS : 1);  // G4: hi_full
     for (int s = 0; s < 2; ++s) {
       mbar_init(&bar_acc_full[s], 1);
       mbar_init(&bar_acc_empty[s], 32 * EPI_WARPS);
@@ -268,7 +317,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) dense_tc_kernel(const DenseArgs
     fence_mbar_init();
   }
   // ---- B operand (weights) resident in shared memory for the whole kernel ----
-  for (int f = tid; f < n_pad * kb16; f += TC_THREADS) {
+  for (int f = tid; f < n_pad * kb16; f += NT) {
     // unit f -> (row group, 16B column): lanes of a quarter warp take the 8 rows of one core matrix
     const int r = ((f >> 3) / kb16) * 8 + (f & 7);
     const int j = (f >> 3) % kb16;
@@ -299,7 +348,65 @@ __global__ void __launch_bounds__(TC_THREADS, 1) dense_tc_kernel(const DenseArgs
   const int64_t n_tiles = a.rows_packed ? (int64_t)*a.n_tiles_dev : (a.M + TM - 1) / TM;
   const int64_t my_tiles = (int64_t)blockIdx.x < n_tiles ? (n_tiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
 
-  if (warp >= EPI_WARPS && warp < EPI_WARPS + LOADER_WARPS) {
+  if (G4 && warp > MMA_WARP) {
+    // ================= TMA producer =================
+    // producer warp pw, lane l < 8 gathers tile rows 32 pw + 4 l .. + 3: row (slot, node) of K chunk kc is row
+    // slot * in_s_stride / 32 + node + kc * in_chunk_stride / 32 of the [rows][32] view.  Rows without an entry read
+    // row 0: the MMA rows are independent and the epilogue stores no row without an entry.  The TMA instructions of one
+    // warp issue one lane after the other; several warps issue side by side.
+    const int pw = warp - (MMA_WARP + 1);
+    if (lane < 8) {
+      const int32_t s_rows = (int32_t)(a.in_s_stride >> 5), c_rows = (int32_t)(a.in_chunk_stride >> 5);
+      auto tile_entries = [&](int64_t ti_) {
+        return __ldg(reinterpret_cast<const int4*>(a.rows_packed + ((int64_t)blockIdx.x + ti_ * gridDim.x) * 128 + pw * 32) + lane);
+      };
+      int4 nxt = my_tiles > 0 ? tile_entries(0) : make_int4(-1, -1, -1, -1);
+      int64_t item = 0;
+      for (int64_t ti = 0; ti < my_tiles; ++ti) {
+        const int e[4] = {nxt.x, nxt.y, nxt.z, nxt.w};
+        int r0[4];
+#pragma unroll
+        for (int p = 0; p < 4; ++p) r0[p] = e[p] < 0 ? 0 : (int32_t)((uint32_t)e[p] >> kPackShift) * s_rows + (e[p] & ((1 << kPackShift) - 1));
+        if (ti + 1 < my_tiles) nxt = tile_entries(ti + 1);  // a tile ahead: in flight while this tile's chunks are issued
+        for (int kc = 0; kc < n_chunks; ++kc, ++item) {
+          const int hs = (int)(item % n_stages);
+          if (item >= n_stages) mbar_wait(&hi_empty[hs], (uint32_t)((item / n_stages) - 1) & 1u);
+          if (lane == 0) mbar_arrive_expect_tx(&hi_full[hs], G4_PART / G4_PROD_WARPS);
+          __syncwarp(0xffu);
+          const int c = kc * c_rows;
+          tma_gather4(smem_u32(sA) + hs * G4_PART + (pw * 8 + lane) * 512, &tmap, r0[0] + c, r0[1] + c, r0[2] + c, r0[3] + c, &hi_full[hs]);
+        }
+      }
+    }
+  } else if (G4 && warp >= EPI_WARPS && warp < MMA_WARP) {
+    // ================= converters =================
+    // thread t owns bytes 16 (t + 64 q), q = 0..15, of the stage: one warp instruction = 512 contiguous bytes (no bank
+    // conflicts); hi and lo stages share the layout, so the swizzle never has to be known here
+    constexpr int CT = 32 * G4_CONV_WARPS;
+    const int t = tid - EPI_WARPS * 32;
+    const int64_t n_items = my_tiles * n_chunks;
+    for (int64_t i = 0; i < n_items; ++i) {
+      const int hs = (int)(i % n_stages), ls = (int)(i % G4_LO);
+      mbar_wait(&hi_full[hs], (uint32_t)(i / n_stages) & 1u);
+      if (i >= G4_LO) mbar_wait(&lo_empty[ls], (uint32_t)((i / G4_LO) - 1) & 1u);
+      const float4* hi = reinterpret_cast<const float4*>(sA + (size_t)hs * G4_PART);
+      float4* lo = reinterpret_cast<float4*>(sA + (size_t)(n_stages + ls) * G4_PART);
+#pragma unroll
+      for (int h8 = 0; h8 < G4_PART / 16 / CT; h8 += 8) {
+        float4 v[8];
+#pragma unroll
+        for (int q = 0; q < 8; ++q) v[q] = hi[t + CT * (h8 + q)];
+#pragma unroll
+        for (int q = 0; q < 8; ++q) {
+          float4 h, l;
+          split_tf32(v[q], h, l);
+          lo[t + CT * (h8 + q)] = l;
+        }
+      }
+      fence_proxy_async();  // generic-proxy stores -> visible to the tensor core (async proxy)
+      mbar_arrive(&bar_full[ls]);
+    }
+  } else if (!G4 && warp >= EPI_WARPS && warp < EPI_WARPS + LOADER_WARPS) {
     // ================= loaders / converters =================
     // LOADER_GROUPS groups of 4 warps take the K chunks round-robin.  A thread has only its own chunk in flight
     // when it executes fence.proxy.async (the fence waits for every outstanding load of the thread: prefetching
@@ -392,7 +499,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) dense_tc_kernel(const DenseArgs
       dbg[0] = (unsigned long long)(clock64() - t_role0);
       dbg[1] = w_empty;
     }
-  } else if (warp == EPI_WARPS + LOADER_WARPS) {
+  } else if (warp == MMA_WARP) {
     // ================= MMA issue (one lane) =================
     if (lane == 0) {
       const uint32_t idesc = make_idesc(MODE == 0 ? 2 : 1, TM, n_pad);
@@ -408,29 +515,37 @@ __global__ void __launch_bounds__(TC_THREADS, 1) dense_tc_kernel(const DenseArgs
         }
         const uint32_t d_tmem = tmem_base + (uint32_t)(ab * n_pad);
         for (int kc = 0; kc < n_chunks; ++kc, ++item) {
-          const int st = (int)(item % n_stages);
-          mbar_wait_timed(&bar_full[st], (uint32_t)(item / n_stages) & 1u, dbg, w_full);
+          const int st = (int)(item % n_stages), ls = (int)(item % G4_LO);
+          if (G4)
+            mbar_wait_timed(&bar_full[ls], (uint32_t)(item / G4_LO) & 1u, dbg, w_full);
+          else
+            mbar_wait_timed(&bar_full[st], (uint32_t)(item / n_stages) & 1u, dbg, w_full);
           tc_fence_after();
-          const uint32_t a_hi = sA_addr + st * Cfg::A_STAGE_BYTES;
-          const uint32_t a_lo = a_hi + Cfg::PART_BYTES;
+          const uint32_t a_hi = sA_addr + st * (G4 ? G4_PART : Cfg::A_STAGE_BYTES);
+          const uint32_t a_lo = G4 ? sA_addr + (n_stages + ls) * G4_PART : a_hi + Cfg::PART_BYTES;
 #pragma unroll
           for (int ks = 0; ks < KC / Cfg::UK; ++ks) {
             // one MMA consumes 2 sixteen-byte columns (32 bytes of K)
-            const uint32_t a_off = ks * 2 * 128;
+            const uint32_t a_off = ks * 2 * (G4 ? 16 : 128);
             const uint32_t b_off = (kc * Cfg::K16 + ks * 2) * 128;
-            const uint64_t da_hi = smem_desc(a_hi + a_off, 128, Cfg::K16 * 128);
+            const uint64_t da_hi = G4 ? smem_desc_sw128(a_hi + a_off) : smem_desc(a_hi + a_off, 128, Cfg::K16 * 128);
             const uint64_t db_hi = smem_desc(sB_addr + b_off, 128, kb16 * 128);
             const uint32_t first = (kc == 0 && ks == 0) ? 0u : 1u;
             if (XP_EXP(a, 4)) continue;
             umma<MODE>(d_tmem, da_hi, db_hi, idesc, first);
             if (MODE == 0) {
-              const uint64_t da_lo = smem_desc(a_lo + a_off, 128, Cfg::K16 * 128);
+              const uint64_t da_lo = G4 ? smem_desc_sw128(a_lo + a_off) : smem_desc(a_lo + a_off, 128, Cfg::K16 * 128);
               const uint64_t db_lo = smem_desc(sB_addr + b_part_bytes + b_off, 128, kb16 * 128);
               umma<MODE>(d_tmem, da_lo, db_hi, idesc, 1u);
               umma<MODE>(d_tmem, da_hi, db_lo, idesc, 1u);
             }
           }
-          umma_commit(&bar_done[item % n_done]);
+          if (G4) {
+            umma_commit(&hi_empty[st]);
+            umma_commit(&lo_empty[ls]);
+          } else {
+            umma_commit(&bar_done[item % n_done]);
+          }
           if (kc == n_chunks - 1) umma_commit(&bar_acc_full[ab]);
         }
       }
@@ -578,6 +693,37 @@ static bool tc_eligible(const DenseArgs& d, int mode) {
   return tc_stages(d, mode) >= 2;
 }
 
+// G4: landed hi stages that fit next to the weights and the G4_LO lo stages (0: the gather4 form does not apply)
+static int g4_stages(const DenseArgs& d) {
+  static int budget = -1;  // dynamic shared memory a CTA of the G4 kernel may use
+  if (budget < 0) {
+    int dev = 0, optin = 0;
+    cudaFuncAttributes fa;
+    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess ||
+        cudaFuncGetAttributes(&fa, dense_tc_kernel<0, true>) != cudaSuccess) {
+      (void)cudaGetLastError();
+      return 0;
+    }
+    budget = optin - (int)fa.sharedSizeBytes - 1024;  // 1024: alignment of the swizzled stages
+  }
+  const int64_t room = (int64_t)budget - (int64_t)tc_b_bytes(d, 0);
+  return (int)std::min<int64_t>(G4_MAX_HI, std::max<int64_t>(room / G4_PART - G4_LO, 0));
+}
+// rows of the [rows][32 floats] view that the tile table can name: slots below ceil(M / slot tiles), nodes below
+// in_chunk_stride / 32 (a chunk holds every node)
+static int64_t g4_rows(const DenseArgs& d) {
+  const int64_t slot_rows = ceil_div((int64_t)d.rows_per_s, (int64_t)TM) * TM;
+  const int64_t n_slots = ceil_div(d.M, slot_rows);
+  return ((n_slots - 1) * d.in_s_stride + (int64_t)(d.k / KC) * d.in_chunk_stride) / 32;
+}
+// TF32x3 with a chunk-major input of 32-float chunks, rows from the tile table: A by TMA gather4 (option dense_tma)
+static bool g4_eligible(const DenseArgs& d, int mode) {
+  if (mode != 0 || !knobs().dense_tma || !d.rows_packed || d.in16 || d.cw_in != 32 || d.ld_in != 32) return false;
+  if (d.in_s_stride % 32 != 0 || d.in_chunk_stride % 32 != 0 || ((uintptr_t)d.in & 15) != 0 || ((uintptr_t)d.rows_packed & 15) != 0) return false;
+  if (g4_rows(d) >= (1ll << 31)) return false;  // gather4 row coordinates are int32
+  return g4_stages(d) >= 2;
+}
+
 int launch_dense_tc(const DenseArgs& d_in, int mode, cudaStream_t st) {
   DenseArgs d = d_in;
 #ifdef XPGNN_EXPERIMENTS  // ablation build only (make EXPERIMENTS=1): never in the shipped library
@@ -601,8 +747,13 @@ int launch_dense_tc(const DenseArgs& d_in, int mode, cudaStream_t st) {
   const int n_pad = (d.n_out + 15) / 16 * 16;
   uint32_t cols = 32;
   while ((int)cols < 2 * n_pad) cols <<= 1;  // two accumulator buffers
-  const int stages = tc_stages(d, mode);
-  const size_t smem = tc_b_bytes(d, mode) + (size_t)stages * (mode == 0 ? TcCfg<0>::A_STAGE_BYTES : TcCfg<1>::A_STAGE_BYTES);
+  const bool g4 = g4_eligible(d, mode);
+  const int stages = g4 ? g4_stages(d) : tc_stages(d, mode);
+  const size_t smem = g4 ? tc_b_bytes(d, mode) + (size_t)(stages + G4_LO) * G4_PART + 1024
+                         : tc_b_bytes(d, mode) + (size_t)stages * (mode == 0 ? TcCfg<0>::A_STAGE_BYTES : TcCfg<1>::A_STAGE_BYTES);
+  CUtensorMap tmap;
+  memset(&tmap, 0, sizeof tmap);
+  if (g4 && rows128_tensor_map(d.in, (uint64_t)g4_rows(d), true, &tmap)) return 1;
   const int64_t tiles = ceil_div(d.M, TM);
   const int grid = (int)std::min<int64_t>(tiles, kNumSMs);
   // XPGNN_DENSE_DBG=1: per-role cycle counters of CTA 0 (synchronises; diagnostics only)
@@ -616,13 +767,10 @@ int launch_dense_tc(const DenseArgs& d_in, int mode, cudaStream_t st) {
     XP_CHECK(cudaMalloc(&dbg, 8 * sizeof(unsigned long long)));
     XP_CHECK(cudaMemsetAsync(dbg, 0, 8 * sizeof(unsigned long long), st));
   }
-  if (mode == 0) {
-    XP_CHECK(cudaFuncSetAttribute(dense_tc_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    XP_LAUNCH(dense_tc_kernel<0>, grid, TC_THREADS, smem, st, d, n_pad, cols, stages, dbg);
-  } else {
-    XP_CHECK(cudaFuncSetAttribute(dense_tc_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    XP_LAUNCH(dense_tc_kernel<1>, grid, TC_THREADS, smem, st, d, n_pad, cols, stages, dbg);
-  }
+  void (*k)(const DenseArgs, int, uint32_t, int, unsigned long long*, const CUtensorMap) =
+      g4 ? dense_tc_kernel<0, true> : (mode == 0 ? dense_tc_kernel<0, false> : dense_tc_kernel<1, false>);
+  XP_CHECK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  XP_LAUNCH(k, grid, g4 ? G4_THREADS : TC_THREADS, smem, st, d, n_pad, cols, stages, dbg, tmap);
   if (dbg_on) {
     unsigned long long h[8];
     XP_CHECK(cudaStreamSynchronize(st));

@@ -37,6 +37,8 @@ struct Knobs {
   int l0_wait_ns = 2000;    // XPGNN_L0_WAIT_NS: the same for the warp-specialised layer-0 kernel
   int dense_wait_ns = 2000;  // XPGNN_DENSE_WAIT_NS: > 0 = waiting warps of dense_tc suspend inside mbarrier.try_wait (hint in ns) instead of polling
                            // (0 = poll + nanosleep; measured 3.94 -> 3.89 ms per C3 tile launch, layer 0 4.96 -> 4.95)
+  int dense_tma = 1;       // XPGNN_DENSE_TMA: TF32x3 transforms of chunk-major 32-float inputs with tile-table rows load A by TMA gather4
+                           // and feed the landed rows to the tensor core as the hi operand (bit-identical; 0: the register loaders)
   int dense_simt = 0;      // XPGNN_DENSE=simt: exact fp32 FMA transforms instead of 3xTF32 tensor-core products
   int prune_l0 = 1;        // XPGNN_PRUNE_L0
   int fused = 0;           // XPGNN_FUSED

@@ -19,7 +19,7 @@ const KnobEntry kKnobTable[] = {
     {"compact", &Knobs::compact}, {"compact_hetero", &Knobs::compact_hetero}, {"cw", &Knobs::cw}, {"l0_lists", &Knobs::l0_lists},
     {"occ", &Knobs::occ}, {"seg", &Knobs::seg}, {"seg_occ", &Knobs::seg_occ}, {"seg_tma", &Knobs::seg_tma}, {"seg_skew", &Knobs::seg_skew}, {"seg_pf", &Knobs::seg_pf}, {"seg_carve", &Knobs::seg_carve}, {"l0_slices", &Knobs::l0_slices}, {"act_column", &Knobs::act_column}, {"l2_stream", &Knobs::l2_stream},
     {"l2_gather", &Knobs::l2_gather}, {"sched_static", &Knobs::sched_static}, {"long_rows", &Knobs::long_rows}, {"occ16", &Knobs::occ16},
-    {"l0_multi", &Knobs::l0_multi}, {"l1_multi", &Knobs::l1_multi}, {"l0_ws", &Knobs::l0_ws}, {"dense_simt", &Knobs::dense_simt}, {"dense_wait_ns", &Knobs::dense_wait_ns}, {"l0_wait_ns", &Knobs::l0_wait_ns},
+    {"l0_multi", &Knobs::l0_multi}, {"l1_multi", &Knobs::l1_multi}, {"l0_ws", &Knobs::l0_ws}, {"dense_simt", &Knobs::dense_simt}, {"dense_wait_ns", &Knobs::dense_wait_ns}, {"dense_tma", &Knobs::dense_tma}, {"l0_wait_ns", &Knobs::l0_wait_ns},
     {"prune_l0", &Knobs::prune_l0}, {"fused", &Knobs::fused}, {"fused_sb", &Knobs::fused_sb}};
 int env_int(const char* name, int dflt) {
   const char* e = getenv(name);
@@ -45,6 +45,7 @@ Knobs& knobs() {
     d.seg_skew = env_int("XPGNN_SEG_SKEW", d.seg_skew);
     d.seg_pf = env_int("XPGNN_SEG_PF", d.seg_pf);
     d.dense_wait_ns = env_int("XPGNN_DENSE_WAIT_NS", d.dense_wait_ns);
+    d.dense_tma = env_int("XPGNN_DENSE_TMA", d.dense_tma);
     d.l0_wait_ns = env_int("XPGNN_L0_WAIT_NS", d.l0_wait_ns);
     d.l0_slices = env_int("XPGNN_L0_SLICES", d.l0_slices);
     d.act_column = env_int("XPGNN_ACT_COLUMN", d.act_column);

@@ -38,7 +38,8 @@ int64_t xpgnn_launch_count(void);
  * variables only seed the defaults and are read ONCE, at the first use of the library; afterwards an option changes
  * only through this call.  Names (csrc/knobs.cuh): compact, compact_hetero, cw, l0_lists, occ, seg, seg_occ, seg_skew, seg_tma,
  * seg_pf, seg_carve, l2_stream, l2_gather, sched_static, long_rows, l0_slices, occ16, l0_multi, l1_multi, l0_ws, l0_wait_ns,
- * dense_wait_ns, dense_simt (1: exact fp32 FMA transforms instead of the 3xTF32 tensor-core products of the fp32 plan),
+ * dense_wait_ns, dense_tma (0: register loaders instead of TMA gather4 for the A operand of the layer >= 1 TF32x3 transforms;
+ * bit-identical), dense_simt (1: exact fp32 FMA transforms instead of the 3xTF32 tensor-core products of the fp32 plan),
  * prune_l0, fused, fused_sb.
  * The reference has no counterpart (its arch call is a black box, model.py:104-112). */
 int xpgnn_set_option(const char* name, int32_t value);
